@@ -48,15 +48,19 @@ __device__ __forceinline__ float4 load_y4(const void* __restrict__ y, int64_t i)
 }
 
 // Per-channel (sum a, sum b, max c) over pixels; thread = one float4 channel group, strided over pixels.
-// Block partials go through shared-memory atomics, then one double atomicAdd per channel per block.
+// Block partials go through shared-memory atomics, then one double atomicAdd per channel per block.  The threads'
+// fp32 partials meet in fp64 (exact while they span fewer than ~29 binary orders of magnitude, otherwise rounded in
+// the last fp64 bits), so the arrival order of the atomics almost never reaches the fp32 statistics.
 template <bool BWD, bool I16 = false>
 __global__ void __launch_bounds__(kBnThreads)
 bn_reduce_kernel(const float4* __restrict__ p0, const void* __restrict__ p1, const float* __restrict__ mean,
                  const float* __restrict__ invstd, int64_t n_pix, int C4, double* __restrict__ sums,
                  uint32_t* __restrict__ maxbits, const float* __restrict__ alpha = nullptr) {
-  extern __shared__ float sh[];               // [3][C]
+  extern __shared__ double sh[];              // [2][C] sums, then [C] max bits (bn_reduce_smem)
   const int C = C4 * 4;
-  for (int i = threadIdx.x; i < 3 * C; i += blockDim.x) sh[i] = 0.f;
+  uint32_t* shm = reinterpret_cast<uint32_t*>(sh + 2 * C);   // non-negative floats order like uints
+  for (int i = threadIdx.x; i < 2 * C; i += blockDim.x) sh[i] = 0.0;
+  for (int i = threadIdx.x; i < C; i += blockDim.x) shm[i] = 0u;
   __syncthreads();
   const int64_t gtid = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
   const int64_t nthreads = int64_t(gridDim.x) * blockDim.x;   // multiple of C4 (host guarantees)
@@ -95,18 +99,28 @@ bn_reduce_kernel(const float4* __restrict__ p0, const void* __restrict__ p1, con
     mx.z = fmaxf(mx.z, fabsf(u.z)); mx.w = fmaxf(mx.w, fabsf(u.w));
   }
   const int c = c4 * 4;
-  atomicAdd(&sh[c + 0], sa.x); atomicAdd(&sh[c + 1], sa.y); atomicAdd(&sh[c + 2], sa.z); atomicAdd(&sh[c + 3], sa.w);
-  atomicAdd(&sh[C + c + 0], sb.x); atomicAdd(&sh[C + c + 1], sb.y);
-  atomicAdd(&sh[C + c + 2], sb.z); atomicAdd(&sh[C + c + 3], sb.w);
-  uint32_t* shm = reinterpret_cast<uint32_t*>(sh + 2 * C);   // non-negative floats order like uints
+  atomicAdd(&sh[c + 0], double(sa.x)); atomicAdd(&sh[c + 1], double(sa.y));
+  atomicAdd(&sh[c + 2], double(sa.z)); atomicAdd(&sh[c + 3], double(sa.w));
+  atomicAdd(&sh[C + c + 0], double(sb.x)); atomicAdd(&sh[C + c + 1], double(sb.y));
+  atomicAdd(&sh[C + c + 2], double(sb.z)); atomicAdd(&sh[C + c + 3], double(sb.w));
   atomicMax(&shm[c + 0], __float_as_uint(mx.x)); atomicMax(&shm[c + 1], __float_as_uint(mx.y));
   atomicMax(&shm[c + 2], __float_as_uint(mx.z)); atomicMax(&shm[c + 3], __float_as_uint(mx.w));
   __syncthreads();
   for (int i = threadIdx.x; i < C; i += blockDim.x) {
-    atomicAdd(sums + i, double(sh[i]));
-    atomicAdd(sums + C + i, double(sh[C + i]));
+    atomicAdd(sums + i, sh[i]);
+    atomicAdd(sums + C + i, sh[C + i]);
     atomicMax(maxbits + i, shm[i]);
   }
+}
+
+// Dynamic shared memory of bn_reduce_kernel: [2][C] fp64 sums + [C] max bits; above the default 48 KB (C > 2457)
+// the kernel has to opt in first.
+static size_t bn_reduce_smem(int C) { return size_t(C) * (2 * sizeof(double) + sizeof(uint32_t)); }
+template <typename Kernel>
+static cudaError_t bn_reduce_allow(Kernel kernel, int C) {
+  return bn_reduce_smem(C) > 48 * 1024
+             ? cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(bn_reduce_smem(C)))
+             : cudaSuccess;
 }
 
 // [C] math of the forward: mean, invstd, a = gamma*invstd, b = beta - mean*a, running statistics
@@ -300,8 +314,9 @@ static int bn_grid(int64_t work, int C4, int per_sm = 8) {
 int bn_stats_launch(const float* y, int64_t n_pix, int C, double* sums, uint32_t* ymax, cudaStream_t st) {
   BDBNN_REQUIRE(C > 0 && (C & 3) == 0 && C <= 4096, "bn_stats: C must be a multiple of 4, <= 4096");
   const int C4 = C / 4;
+  BDBNN_CUDA(bn_reduce_allow(bn_reduce_kernel<false>, C));
   bn_reduce_kernel<false><<<bn_grid(n_pix * C4 / 8, C4, n_pix * C4 > (int64_t(16) << 20) ? 8 : 3), kBnThreads,
-                            size_t(3 * C) * sizeof(float), st>>>(reinterpret_cast<const float4*>(y), nullptr, nullptr,
+                            bn_reduce_smem(C), st>>>(reinterpret_cast<const float4*>(y), nullptr, nullptr,
                                                                  nullptr, n_pix, C4, sums, ymax);
   return check_launch("bn_reduce_kernel<fwd>");
 }
@@ -411,11 +426,12 @@ static int bn_bwd_pack_impl(const float* gz, const void* y, const float* alpha_i
     BDBNN_CUDA(cudaMemsetAsync(sums_ws, 0, size_t(2 * C) * sizeof(double), st));
     BDBNN_CUDA(cudaMemsetAsync(gmax_bits, 0, size_t(C) * sizeof(uint32_t), st));
     const int rgrid = bn_grid(n_pix * C4 / 8, C4, n_pix * C4 > (int64_t(16) << 20) ? 8 : 3);
+    BDBNN_CUDA(i16 ? bn_reduce_allow(bn_reduce_kernel<true, true>, C) : bn_reduce_allow(bn_reduce_kernel<true, false>, C));
     if (i16)
-      bn_reduce_kernel<true, true><<<rgrid, kBnThreads, size_t(3 * C) * sizeof(float), st>>>(
+      bn_reduce_kernel<true, true><<<rgrid, kBnThreads, bn_reduce_smem(C), st>>>(
           reinterpret_cast<const float4*>(gz), y, mean, invstd, n_pix, C4, sums_ws, gmax_bits, alpha_i16);
     else
-      bn_reduce_kernel<true, false><<<rgrid, kBnThreads, size_t(3 * C) * sizeof(float), st>>>(
+      bn_reduce_kernel<true, false><<<rgrid, kBnThreads, bn_reduce_smem(C), st>>>(
           reinterpret_cast<const float4*>(gz), y, mean, invstd, n_pix, C4, sums_ws, gmax_bits, nullptr);
     rc = check_launch("bn_reduce_kernel<bwd>");
     if (rc) return rc;
@@ -838,7 +854,8 @@ extern "C" int bdbnn_bn_pool_bwd(const float* g_pool, const uint8_t* idx, const 
   const int64_t n_pool = int64_t(N) * Ho * Wo, n_full = int64_t(N) * H * W;
   BDBNN_CUDA(cudaMemsetAsync(sums_ws, 0, size_t(2 * C) * sizeof(double), st));
   BDBNN_CUDA(cudaMemsetAsync(gmax_bits, 0, size_t(C) * sizeof(uint32_t), st));
-  bn_reduce_kernel<true><<<bn_grid(n_pool * C4 / 8, C4, 3), kBnThreads, size_t(3 * C) * sizeof(float), st>>>(
+  BDBNN_CUDA(bn_reduce_allow(bn_reduce_kernel<true>, C));
+  bn_reduce_kernel<true><<<bn_grid(n_pool * C4 / 8, C4, 3), kBnThreads, bn_reduce_smem(C), st>>>(
       reinterpret_cast<const float4*>(g_pool), reinterpret_cast<const float4*>(y_sel), mean, invstd, n_pool, C4,
       sums_ws, gmax_bits);
   rc = check_launch("bn_reduce_kernel<bwd,pool>");

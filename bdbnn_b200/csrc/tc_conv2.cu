@@ -124,13 +124,17 @@ tc_conv2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
   __shared__ __align__(8) uint64_t tfull_bar[2], tempty_bar[2];
   __shared__ uint32_t tmem_slot;
   __shared__ uint32_t tap_shift_rows[kMaxTaps];   // halo: row offset of tap i inside the patch
-  // BatchNorm statistics of this CTA's output rows (MODE 0 with p.bn_sums): fp32 partials, flushed once
+  // BatchNorm statistics of this CTA's output rows (MODE 0 with p.bn_sums), flushed once.  The warps' fp32 partials
+  // meet in fp64, where their sum is exact while they span fewer than ~29 binary orders of magnitude, and otherwise
+  // rounds in the last fp64 bits only: the order the atomics arrive in (and the order of the per-CTA fp64 atomics
+  // below) then almost never reaches the fp32 mean / variance.  fp32 shared atomics changed those in the last bit
+  // from run to run, and in a binarised network a last-bit difference flips signs downstream.
   constexpr bool kStats = MODE == 0 || BST;
-  __shared__ float stat_sum[kStats ? kMaxStatCh : 1], stat_sq[kStats ? kMaxStatCh : 1];
+  __shared__ double stat_sum[kStats ? kMaxStatCh : 1], stat_sq[kStats ? kMaxStatCh : 1];
   __shared__ uint32_t stat_max[kStats ? kMaxStatCh : 1];
   const bool do_stats = kStats && p.bn_sums != nullptr;   // MODE 0: statistics of y; MODE 1 (BST): backward statistics of gz
   if (do_stats)
-    for (int i = threadIdx.x; i < p.Nout; i += blockDim.x) { stat_sum[i] = 0.f; stat_sq[i] = 0.f; stat_max[i] = 0u; }
+    for (int i = threadIdx.x; i < p.Nout; i += blockDim.x) { stat_sum[i] = 0.0; stat_sq[i] = 0.0; stat_max[i] = 0u; }
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   if (threadIdx.x < p.n_taps)
@@ -349,10 +353,10 @@ tc_conv2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
         }
         if (lane < 8) {
           const int ch = acc_nn0 + cb * 32 + lane * 4;
-          atomicAdd(&stat_sum[ch], ss.x); atomicAdd(&stat_sum[ch + 1], ss.y);
-          atomicAdd(&stat_sum[ch + 2], ss.z); atomicAdd(&stat_sum[ch + 3], ss.w);
-          atomicAdd(&stat_sq[ch], sq.x); atomicAdd(&stat_sq[ch + 1], sq.y);
-          atomicAdd(&stat_sq[ch + 2], sq.z); atomicAdd(&stat_sq[ch + 3], sq.w);
+          atomicAdd(&stat_sum[ch], double(ss.x)); atomicAdd(&stat_sum[ch + 1], double(ss.y));
+          atomicAdd(&stat_sum[ch + 2], double(ss.z)); atomicAdd(&stat_sum[ch + 3], double(ss.w));
+          atomicAdd(&stat_sq[ch], double(sq.x)); atomicAdd(&stat_sq[ch + 1], double(sq.y));
+          atomicAdd(&stat_sq[ch + 2], double(sq.z)); atomicAdd(&stat_sq[ch + 3], double(sq.w));
           atomicMax(&stat_max[ch], __float_as_uint(mx.x)); atomicMax(&stat_max[ch + 1], __float_as_uint(mx.y));
           atomicMax(&stat_max[ch + 2], __float_as_uint(mx.z)); atomicMax(&stat_max[ch + 3], __float_as_uint(mx.w));
         }
@@ -527,9 +531,9 @@ tc_conv2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
   if (do_stats) {
     // one fp64 atomic per channel per CTA; channels this CTA never touched hold zeros
     for (int i = threadIdx.x; i < p.Nout; i += blockDim.x) {
-      if (stat_max[i] != 0u || stat_sum[i] != 0.f || stat_sq[i] != 0.f) {
-        atomicAdd(p.bn_sums + i, double(stat_sum[i]));
-        atomicAdd(p.bn_sums + p.Nout + i, double(stat_sq[i]));
+      if (stat_max[i] != 0u || stat_sum[i] != 0.0 || stat_sq[i] != 0.0) {
+        atomicAdd(p.bn_sums + i, stat_sum[i]);
+        atomicAdd(p.bn_sums + p.Nout + i, stat_sq[i]);
         atomicMax(p.bn_ymax + i, stat_max[i]);
       }
     }
@@ -689,9 +693,9 @@ int launch_tc_conv2(const TcConvLaunch& L, int mode, cudaStream_t st) {
   if (rc) return rc;
   const uint32_t kStaging = uint32_t(kEpiWarps) * 4096u;   // epilogue transpose tiles
   const uint32_t fixed = (p.halo ? 2u * p.patch_bytes : 0u) + kStaging;
-  // 227 KB per CTA minus static shared memory (barriers; MODE 0 also holds 6 KB of BN statistics)
+  // 227 KB per CTA minus static shared memory (barriers; MODE 0 also holds 10 KB of BN statistics)
   const bool bst = mode == 1 && p.bn_sums != nullptr;
-  const uint32_t budget = 224u * 1024u - 1024u - ((mode == 0 || bst) ? 3u * kMaxStatCh * 4u : 0u);
+  const uint32_t budget = 224u * 1024u - 1024u - ((mode == 0 || bst) ? (2u * 8u + 4u) * kMaxStatCh : 0u);
   if (fixed + 2u * p.stage_bytes > budget) return BDBNN_ERR_UNSUPPORTED;
   int stages = int((budget - fixed) / p.stage_bytes);
   if (stages > kMaxStages) stages = kMaxStages;

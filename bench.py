@@ -4,6 +4,7 @@
     python bench.py --gpus 1 --steps 20 --warmup 5            # this repo (CUDA kernels)
     torchrun ... bench.py --gpus N --steps K --warmup W       # one rank per GPU, NCCL
     python bench.py --impl reference ...                      # reference arm: the CPU oracle step
+    python bench.py --gpus 1 --steps 20 --warmup 5 --dump-outputs DIR   # + the last timed step's outputs as .npy
 
 A "step" = one full optimisation step of the restated train.py body (bdbnn_b200.step.TrainStep:
 forward, losses, backward, gradient all-reduce, optimizer) on one synthetic batch.  Workload at N=1 is
@@ -56,7 +57,14 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--profile-mode", action="store_true",
                     help="for runs under ncu: 1 warm-up step, no e2e / cpu legs (numbers printed are not bench values)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of --impl b200")
+    return args
 
 
 TRAFFIC_KERNEL = {  # KernelTimer family -> kernel-name prefixes in profiles/*_dram_traffic.json (ncu --set full)
@@ -153,6 +161,40 @@ class ClockSampler:
                     reasons.add(nm)
         return {"sm_mhz": statistics.median(sm) if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "power_w_max": max(pw) if pw else None, "samples": len(sm), "reasons": sorted(reasons)}
+
+
+DUMP_BYTES = 60 << 20          # all arrays of --dump-outputs together, under 64 MB with the .npy headers
+
+
+def dump_outputs(dirname, out, model):
+    """Write what one training step computed as DIR/<name>.npy: every tensor the step returns (`loss`, `ce`,
+    `acc1`, `acc5`, the logits as `output`, and the kurtosis / KD terms when they are on) and the floating-point
+    state the step updated (`model.<state_dict name>`, parameters and BatchNorm statistics, in their logical
+    NCHW / OIHW order).  float64 stays float64, everything else is written as float32.  When the whole set would
+    exceed DUMP_BYTES, every array above an equal share of what is left is cut to a fixed sample of its flattened
+    elements: the first k positions of a permutation seeded with 0, in ascending order.  With the same arguments
+    the inputs are the same on every run.  So are the outputs of the default ResNet-18 CE workload, which runs no
+    cuDNN (tests/test_gpu_step.py repeats three such steps bit for bit); workloads that run
+    cuDNN under cudnn.benchmark=True (the kurt_kd teacher, the ResNet-20 stem) may time their way to another
+    algorithm on another run and then differ."""
+    import numpy as np
+    arrays = {k: v for k, v in out.items() if torch.is_tensor(v)}
+    arrays.update({f"model.{k}": v for k, v in model.state_dict().items() if v.is_floating_point()})
+    arrays = {k: v.detach().to("cpu", torch.float64 if v.dtype == torch.float64 else torch.float32).contiguous()
+              for k, v in arrays.items()}
+    nbytes = lambda t: t.numel() * t.element_size()
+    left, cap = DUMP_BYTES, None
+    for i, v in enumerate(sorted(arrays.values(), key=nbytes)):       # smallest first: each takes at most its share
+        if nbytes(v) > left // (len(arrays) - i):
+            cap = left // (len(arrays) - i)
+            break
+        left -= nbytes(v)
+    os.makedirs(dirname, exist_ok=True)
+    for k, v in arrays.items():
+        if cap is not None and nbytes(v) > cap:
+            keep = torch.randperm(v.numel(), generator=torch.Generator().manual_seed(0))[:cap // v.element_size()]
+            v = v.reshape(-1)[keep.sort().values]
+        np.save(os.path.join(dirname, f"{k}.npy"), v.numpy())
 
 
 def build_model(name, conv_impl=None, ref=False):
@@ -468,7 +510,7 @@ def main():
     sampler.mark_begin()
     e0.record()
     for _ in range(args.steps):
-        step(x_dev, y_dev)
+        out = step(x_dev, y_dev)
     e1.record()
     barrier()
     sampler.mark_end()
@@ -477,6 +519,8 @@ def main():
         torch.cuda.profiler.stop()
     ms_total = max_over_ranks(e0.elapsed_time(e1))
     launches = _lib.launch_count() - n0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out, model)     # before the legs below take further steps on the model
     if use_graph:
         # per-kernel CUDA events cannot be recorded inside a graph: the roofline figures come from the SAME step
         # launched eagerly (identical kernels, identical arguments) right after the timed region

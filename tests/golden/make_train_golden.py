@@ -1,5 +1,5 @@
 """Generate whole-step golden fixtures by executing the REFERENCE's own `train()` and
-`train_teacher_student()` (/root/reference/train.py:441-554, 556-675), imported unmodified through
+`train_teacher_student()` (train.py:441-554, 556-675), imported unmodified through
 tests/ref_launcher.py in "reference" mode: train.py, kurtosis.py, utils/utils.py and utils/KD_loss.py are
 the reference's files; only the `models` package (absent upstream) and the network under test (oracle
 modules, CPU) come from this repo.  Build container only.
@@ -69,5 +69,6 @@ def run_case(case):
 
 
 if __name__ == "__main__":
+    torch.set_num_threads(TC.CPU_THREADS)
     for name in (sys.argv[1:] or TC.CASES):
         run_case(name)

@@ -1,4 +1,4 @@
-"""GPU, 2 ranks over NCCL (run with `gpurun --gpus 2`; skipped when fewer than 2 devices are visible):
+"""GPU, 2 ranks over NCCL (skipped when fewer than 2 devices are visible):
 the product's data-parallel path — GradAllReduce's post-accumulate hooks issuing async bucket all-reduces
 from the autograd thread into the flat .grad views, 1/world folded into FusedAdam (train.py:304, 527-529).
 
@@ -90,7 +90,7 @@ def _single(outdir, init_flat):
     return torch.cat([p.grad.reshape(-1) for p in m.parameters()]).cpu()
 
 
-@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs (gpurun --gpus 2)")
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs")
 @pytest.mark.parametrize("use_shim", [True, False])
 def test_nccl_world2_grads_and_params_identical_and_match_single_process(tmp_path, use_shim):
     import torch.multiprocessing as mp

@@ -11,7 +11,6 @@ Tolerances (whole network, looser than the per-kernel tests): a handful of activ
 round-off of 0 or +-1 take the other sign / STE-mask value on the GPU (different BatchNorm summation
 order), a discrete difference that propagates; gradients are compared relative to max|reference| per tensor."""
 import json
-import os
 
 import pytest
 import torch
@@ -126,7 +125,7 @@ def _metrics(got, ref):
 
 
 @pytest.mark.parametrize("mode", ["fp16s", "bf16x2"])
-def test_gpu_resnet18_224_blockwise_teacher_forced(mode, monkeypatch):
+def test_gpu_resnet18_224_blockwise_teacher_forced(mode, monkeypatch, tmp_path):
     """The code path the headline times (ResNet-18, 224x224: tcgen05 stem + fused BN/pool, fp8 forward, fused
     conv-BN-add units with int16 y, in-node 1x1 shortcuts, classifier), checked block by block against the oracle
     with TEACHER FORCING: every product block receives the oracle's input of that block and the oracle's gradient
@@ -172,8 +171,8 @@ def test_gpu_resnet18_224_blockwise_teacher_forced(mode, monkeypatch):
         for pn, p in params.items():
             m[pn] = _metrics(p.grad, ref_params[pn].grad)
         report[name] = m
-    os.makedirs("gpurun_out", exist_ok=True)
-    with open(f"gpurun_out/r18_blockwise_{mode}.json", "w") as fh:
+    # the per-block error record (profiles/r2_parity_r18_blockwise_*.json); `pytest --basetemp DIR` keeps it
+    with open(tmp_path / f"r18_blockwise_{mode}.json", "w") as fh:
         json.dump(report, fh, indent=1)
     bad = []
     for name, m in report.items():

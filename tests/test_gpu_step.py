@@ -75,3 +75,28 @@ def test_resnet20_step_matches_cpu_oracle(ts, ede):
         scale = gr[n].abs().max().item() + 1e-12
         err = (gg[n] - gr[n]).abs().max().item()
         assert err <= 2e-2 * scale, (n, err, scale)
+
+
+def test_resnet18_steps_are_bit_reproducible():
+    """The same inputs give the same steps, bit for bit.  In a binarised network a last-bit difference flips signs
+    and grows over the following steps; BatchNorm statistics combined through fp32 atomics differed in the last bit
+    from run to run (2 % of max|logit| after one step).  The fp64 combine leaves order effects in the last fp64 bits,
+    which the fp32 statistics almost never see."""
+    from bdbnn_b200.resnet import resnet18
+    from bdbnn_b200.step import StepConfig, TrainStep, make_optimizer
+    g = torch.Generator().manual_seed(0)
+    x = torch.randn(64, 3, 224, 224, generator=g).cuda().contiguous(memory_format=torch.channels_last)
+    y = torch.randint(0, 1000, (64,), generator=g).cuda()
+    runs = []
+    for _ in range(2):
+        torch.manual_seed(0)
+        m = resnet18().cuda()
+        step = TrainStep(m, make_optimizer(m, "imagenet"), StepConfig())
+        outs = [{k: v.clone() for k, v in step(x, y).items() if torch.is_tensor(v)} for _ in range(3)]
+        torch.cuda.synchronize()
+        runs.append((outs, {k: v.clone() for k, v in m.state_dict().items()}))
+    for a, b in zip(runs[0][0], runs[1][0]):
+        for k in a:
+            assert torch.equal(a[k], b[k]), k
+    for k, v in runs[0][1].items():
+        assert torch.equal(v, runs[1][1][k]), k

@@ -351,3 +351,30 @@ def test_bench_reference_arm_prints_the_contract_line():
     assert d["impl"] == "reference" and d["metric"] == "images/sec" and d["higher_is_better"] is True
     assert d["cpu_baseline"]["kind"] == "port" and d["cpu_baseline"]["cores"] >= 1 and d["value"] > 0
     assert d["e2e"]["h2d_bytes_per_step"] == 0 and d["e2e"]["d2h_bytes_per_step"] == 0
+
+
+def test_bench_dump_outputs_writes_the_step_outputs_within_budget(tmp_path, monkeypatch):
+    """`bench.py --dump-outputs`: every returned tensor and every floating-point state entry as <name>.npy (float64
+    kept, the rest float32, shapes kept); above the byte budget, the largest arrays become the same seeded sample
+    of their flattened elements on every run."""
+    import numpy as np
+    import bench
+    torch.manual_seed(0)
+    m = bench.build_model("resnet20", ref=True)
+    out = {"loss": torch.tensor(2.5), "acc1": torch.tensor(50.0, dtype=torch.float64), "kurt": 0,
+           "output": torch.randn(8, 10, dtype=torch.float16)}
+    bench.dump_outputs(str(tmp_path / "all"), out, m)
+    names = {f[:-4] for f in os.listdir(tmp_path / "all")}
+    assert names == {"loss", "acc1", "output"} | {f"model.{k}" for k, v in m.state_dict().items() if v.is_floating_point()}
+    assert np.load(tmp_path / "all" / "acc1.npy").dtype == np.float64 and np.load(tmp_path / "all" / "loss.npy").shape == ()
+    assert np.array_equal(np.load(tmp_path / "all" / "output.npy"), out["output"].float().numpy())
+    w = m.state_dict()["layer3.0.conv2.weight"]
+    assert np.array_equal(np.load(tmp_path / "all" / "model.layer3.0.conv2.weight.npy"), w.numpy())
+    monkeypatch.setattr(bench, "DUMP_BYTES", 64 << 10)
+    for d in ("cut", "cut2"):
+        bench.dump_outputs(str(tmp_path / d), out, m)
+    sizes = {f: np.load(tmp_path / "cut" / f).nbytes for f in os.listdir(tmp_path / "cut")}
+    assert sum(sizes.values()) <= 64 << 10 and sizes["loss.npy"] == 4
+    cut = np.load(tmp_path / "cut" / "model.layer3.0.conv2.weight.npy")
+    assert cut.ndim == 1 and 0 < cut.size < w.numel() and set(cut.tolist()) <= set(w.reshape(-1).tolist())
+    assert np.array_equal(cut, np.load(tmp_path / "cut2" / "model.layer3.0.conv2.weight.npy"))

@@ -24,6 +24,9 @@ CASES = {
 }
 SUMMARY_ONLY = ("r18_ce", "r18_kurt_ts")      # 11.7 M parameters: store per-parameter summaries, not tensors
 N_SAMPLES = 64
+# intra-op threads of every fp32 CPU step that makes or replays a fixture: oneDNN splits its convolution reductions
+# by thread count, and the replay tolerances (1e-6 of max|reference|) hold for the summation order of this count
+CPU_THREADS = 8
 
 
 def build_oracle(case, seed=0):
